@@ -309,6 +309,13 @@ class PpoBench(object):
         if ev: ev[3].record()
         return loss
 
+    def outputs(self):
+        """What the last device_iteration handed its caller: sampled actions, log-probs and values [T, E], GAE advantages
+        and value targets [E*T], the loss of every SGD step and the trained weights."""
+        st, n = self.store, self.n
+        return dict(action=self.act_t, logp=self.logp_t, value=self.val_t[:self.T], adv=st.adv[:n], target_v=st.target_v[:n],
+                    loss=self.model.last_losses, weights=self.model.get_weights())
+
     def e2e_setup(self):
         E, T, ro = self.E, self.T, self.ro
         self.host_obs = [np.ascontiguousarray(ro["obs"][np.arange(E) * T + t]) for t in range(T)]
@@ -375,6 +382,11 @@ class ImpalaBench(object):
         if ev: ev[3].record()
         return self.loss
 
+    def outputs(self):
+        """Sampled actions, log-probs and values [T, E] of the last iteration, the loss of its last SGD step and the
+        trained weights."""
+        return dict(action=self.act_t, logp=self.logp_t, value=self.val_t, loss=self.loss, weights=self.model.get_weights())
+
     def e2e_setup(self):
         E, T, ro = self.E, self.T, self.ro
         self.host_obs = [np.ascontiguousarray(ro["obs"][np.arange(E) * T + t]) for t in range(T)]
@@ -436,6 +448,10 @@ class DqnBench(object):
         if ev: ev[3].record()
         return self.loss
 
+    def outputs(self):
+        """Greedy actions [E] of the last inference call, the loss of the last SGD step and the trained weights."""
+        return dict(action=self.act, loss=self.loss, weights=self.model.get_weights())
+
     def e2e_setup(self):
         tr = self.tr
         self.host_obs = [np.ascontiguousarray(tr["obs"][t * self.E:(t + 1) * self.E]) for t in range(4)]
@@ -450,6 +466,29 @@ class DqnBench(object):
         for s in range(self.steps):
             loss = self.alg.train()
         return loss
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output as <out_dir>/<name>.npy: float64 stays float64, everything else becomes float32 (the integer
+    outputs are small indices, exact in float32).  A weight dict is written as one array, its tensors flattened and
+    concatenated in parameter order."""
+    arrays = {}
+    for name, x in outputs.items():
+        if isinstance(x, dict):
+            x = np.concatenate([np.asarray(v).ravel() for v in x.values()])
+        elif hasattr(x, "cpu"):
+            x = x.cpu().numpy()
+        x = np.asarray(x)
+        arrays[name] = x.astype(np.float64 if x.dtype == np.float64 else np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_b200(args):
@@ -467,6 +506,7 @@ def run_b200(args):
     dev = torch.device("cuda", local)
     wl = WORKLOADS[args.workload]
     comm = engine.GradComm(device=dev) if world > 1 else None          # before the model: graphs are keyed on it
+    np.random.seed(1234 + rank)            # the models draw their action-sampling seed from numpy's global stream
     bench = {"ppo": PpoBench, "impala": ImpalaBench, "dqn": DqnBench}[wl["kind"]](wl, rank, world, dev, local)
     model = bench.model
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)    # > 126 MB L2
@@ -494,6 +534,8 @@ def run_b200(args):
         bench.device_iteration()
         ev[i][1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bench.outputs())
     ms_local = sum(a.elapsed_time(b) for a, b in ev)
     launches = lib.xtb_launch_count() - launches0
     replays = lib.xtb_graph_replay_count() - replays0
@@ -638,7 +680,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="ppo", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0, b200 arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)

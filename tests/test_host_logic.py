@@ -22,12 +22,19 @@ def test_library_builds_loads_and_exports_every_declared_symbol(repo_root):
     raw = C.CDLL(capi.LIB_PATH)
     for name in declared:
         getattr(raw, name)          # raises AttributeError if the .so does not export it
-    assert lib.xtb_launch_count() == 0
+    # a freshly loaded library has launched nothing (this process may already have run kernels in other tests)
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, "-c", "from xingtian_b200 import capi; print(capi.lib().xtb_launch_count())"],
+                         env=dict(os.environ, PYTHONPATH=repo_root), capture_output=True, text=True, timeout=300, cwd=repo_root)
+    assert out.stdout.split() == ["0"], (out.stdout, out.stderr[-500:])
+    launches = lib.xtb_launch_count()
     # argument validation happens before any CUDA call
     assert lib.xtb_gae(None, None, None, 1, 1, 0.99, 0.95, 0, None, None, None, None) == -1
     assert b"null" in lib.xtb_last_error()
     assert lib.xtb_copy_h2d_staged(None, None, 16, None) == -1      # argument check happens before any CUDA call
     assert lib.xtb_ppo_predict_host(None, None, 0, None, 1, 1, 2, 0, None, None, None, 0, None) == -1
+    assert lib.xtb_launch_count() == launches
 
 
 def test_product_has_no_oracle_or_cpu_fallback(repo_root):
